@@ -46,7 +46,7 @@ WORKLOADS = {
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=200)
+    ap.add_argument("--steps", type=int, default=None, help="timed steps (default: 200; loop_batch: 5 passes of the whole batch)")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--workload", default=None, choices=list(WORKLOADS) + ["loop_batch", "voxelgrid", "kitti_pipeline"],
@@ -59,6 +59,8 @@ def parse():
     ap.add_argument("--no-anchor", action="store_true", help="N = 1 odometry line: skip the loop_batch_n1 / strict-chain extras")
     ap.add_argument("--no-profile", action="store_true")
     ap.add_argument("--no-prefetch", action="store_true", help="strict call-by-call chain: do not announce the next frame (no software pipelining)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="odometry workloads: after the timed steps, write what the last timed step returned as DIR/<name>.npy")
     return ap.parse_args()
 
 
@@ -371,6 +373,14 @@ def whole_step_algorithmic_gbs(calls, n, m, stride_bytes, total_ms, steps):
     return total / (total_ms * 1e-3) / 1e9, total / steps, unknown
 
 
+def dump_outputs(out_dir, outputs):
+    """One out_dir/<name>.npy per value a caller of the timed path received: float32 arrays as returned, everything else as float64."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, v in outputs.items():
+        a = np.asarray(v)
+        np.save(os.path.join(out_dir, f"{name}.npy"), a if a.dtype == np.float32 else a.astype(np.float64))
+
+
 def run_b200(args, wl, rank, world, local_rank):
     import torch
     import torch.distributed as dist
@@ -461,7 +471,7 @@ def run_b200(args, wl, rank, world, local_rank):
             sampler.hold(lambda k: step(W + 1 + (k % K)), reg.synchronize)
             clocks = sampler.stop()
         results[arm] = dict(ms=float(t.item()), per_rank_ms=per_rank, wall_ms=wall * 1e3, stats=stats, iters=iters, conv=conv, kf=kf, clocks=clocks,
-                            last_odom=st["odom"])
+                            last=st)
         odo.close()
         reg.close()
 
@@ -470,6 +480,8 @@ def run_b200(args, wl, rank, world, local_rank):
             dist.destroy_process_group()
         return
     rv, re_ = results["value"], results["e2e"]
+    if args.dump_outputs:  # matching_error / inlier_fraction are left out: NaN, as the chain runs without publish_status
+        dump_outputs(args.dump_outputs, {k: v for k, v in rv["last"].items() if k not in ("matching_error", "inlier_fraction")})
     value = world * K / (rv["ms"] * 1e-3)
     e2e = world * K / (re_["ms"] * 1e-3)
     launches = int(sum(rv["stats"]["launches"].values()))
@@ -559,12 +571,14 @@ def main():
     if args.workload is None:
         # the odometry chain cannot shard (frame k's guess is frame k-1's pose): at N > 1 measure the path that does
         args.workload = "loop_batch" if max(world, args.gpus) > 1 else "gicp_odometry_vlp16_64k"
+    if args.dump_outputs and (args.impl != "b200" or args.workload not in WORKLOADS):
+        sys.exit(f"--dump-outputs is implemented for the B200 arm of the odometry workloads ({', '.join(WORKLOADS)})")
+    if args.steps is None:
+        args.steps = 5 if (args.workload, args.impl) == ("loop_batch", "b200") else 200  # loop_batch: 5 timed passes of the whole batch
     if args.workload == "loop_batch":
         if args.impl == "reference":
             return run_reference_loop(args, rank)
         from hdl_graph_slam_b200 import batch
-        if args.steps == 200:
-            args.steps = 5  # default: 5 timed passes of the whole batch
         args.warmup = max(args.warmup, 3) if args.warmup != 5 else 3
         return batch.bench_loop_batch(args, rank, world, local_rank)
     if args.workload in ("voxelgrid", "kitti_pipeline"):

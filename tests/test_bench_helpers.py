@@ -32,6 +32,17 @@ def test_whole_step_algorithmic_throughput():
     assert b.whole_step_algorithmic_gbs(calls, n, n, 32, 0.0, 200) is None
 
 
+def test_dump_outputs_writes_float32_or_float64(tmp_path):
+    import numpy as np
+    b = _bench()
+    T = np.arange(16, dtype=np.float32).reshape(4, 4)
+    b.dump_outputs(str(tmp_path / "d"), {"odom": T, "iterations": 7, "converged": True})
+    assert sorted(os.listdir(tmp_path / "d")) == ["converged.npy", "iterations.npy", "odom.npy"]
+    odom, it, conv = (np.load(tmp_path / "d" / f"{k}.npy") for k in ("odom", "iterations", "converged"))
+    assert odom.dtype == np.float32 and np.array_equal(odom, T)
+    assert it.dtype == np.float64 and it == 7.0 and conv.dtype == np.float64 and conv == 1.0
+
+
 def test_reference_arm_line_has_the_contract_keys(oracle, synth):
     """`bench.py --impl reference` (the CPU oracle replaying the same workload) prints ONE JSON line with the driver's keys"""
     import json
